@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — RepSurf-U fwd+bwd(+SGD step) throughput on synthetic clouds, one process per GPU.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload seg|cls] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload seg|cls] [--impl reference] [--dump-outputs DIR]
 
 Prints ONE JSON line (rank 0).  Contract: see the task statement / DESIGN.md "Measurement".
   value         clouds/sec, whole job, inputs already resident in HBM
@@ -9,8 +9,13 @@ Prints ONE JSON line (rank 0).  Contract: see the task statement / DESIGN.md "Me
                 inputs and D2H of the loss inside the timed region
   roofline      the dominant repsurf_b200 kernel, timed with CUDA events inside the timed region
   cpu_baseline  the oracle port (oracle/model_ref.py + oracle C) on the host cores, bounded sample
-  --impl reference   times that CPU port alone (the reference has no CPU path for segmentation and
-                     /root/reference does not exist on the GPU box; see DESIGN.md)
+  --impl reference   times that CPU port alone (the reference has no CPU path for segmentation; see DESIGN.md)
+  --dump-outputs DIR after the timed steps (rank 0), what the last timed step of each workload returned to its caller:
+                     DIR/<workload>_loss.npy, and the gradients and updated parameters, flattened in parameters() order,
+                     as DIR/<workload>_grads.npy / DIR/<workload>_params.npy (float32).  Model, optimizer and random
+                     state are reset to their seeded initial values before the last timed step, so that the dumped step
+                     does not depend on the steps before it (how many warm-up steps ran, float atomics in their backward):
+                     two builds given the same arguments compute the same step.
 """
 import argparse
 import json
@@ -288,9 +293,13 @@ def gemm_desc(name, a):
     return f"rows={a[0]} K={a[2].K} N={a[1]}, operand kind {a[2].kind}"
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
 def run_ours(workload, args, rank, local_rank, world, dev, full):
     """Times `workload` (value: inputs resident; e2e: pinned host inputs + loss read-back).  full: also the per-entry
-    rooflines, launch count and clocks (primary workload only)."""
+    rooflines, launch count and clocks (primary workload only).  With --dump-outputs, res["outputs"] holds what the last
+    timed step returned (loss, gradients, updated parameters)."""
     import torch.distributed as dist
     from repsurf_b200 import _native
     from repsurf_b200.models import RepSurfCls, RepSurfSeg, SmoothClsLoss
@@ -308,6 +317,7 @@ def run_ours(workload, args, rank, local_rank, world, dev, full):
         crit = SmoothClsLoss()
     params = [p for p in model.parameters()]
     broadcast_module(model)
+    initial_state = {k: v.detach().clone() for k, v in model.state_dict().items()} if args.dump_outputs else None
     # gradients are packed into one flat buffer after backward: ONE all-reduce per step (3.9 MB seg / 5.9 MB cls)
     fg = FlatGrads(params)
     opt = torch.optim.SGD(params, lr=1e-3, momentum=0.9, weight_decay=1e-4)
@@ -363,10 +373,15 @@ def run_ours(workload, args, rank, local_rank, world, dev, full):
     def step_eager():
         return fwd_bwd(devin)
 
+    last = {}
+
     def step_resident():
         if gstep is not None:
-            return gstep(gstep.static_in, gstep.static_tgt)
-        return fwd_bwd(devin)
+            loss = gstep(gstep.static_in, gstep.static_tgt)
+        else:
+            loss = fwd_bwd(devin)
+        last["loss"] = loss
+        return loss
 
     def step_e2e():
         if gstep is not None:                                # pinned host -> the graph's static buffers -> replay -> loss read
@@ -386,7 +401,7 @@ def run_ours(workload, args, rank, local_rank, world, dev, full):
 
     host_issue = {}
 
-    def timed(fn, steps, on_start=None):
+    def timed(fn, steps, on_start=None, before_last=None):
         # the host needs ~12 of a step's ~20 ms to issue it: a full (generation-2) pass of Python's cyclic garbage collector
         # inside the 10-step region (tens of ms over the autograd graphs of a step) makes those steps host-bound - seen twice
         # as a 22 / 33 ms first pass.  Collect before, keep the collector off while timing (reference counting still frees).
@@ -406,7 +421,9 @@ def run_ours(workload, args, rank, local_rank, world, dev, full):
         t0 = time.perf_counter()
         e0.record()
         marks = []
-        for _ in range(steps):
+        for i in range(steps):
+            if before_last is not None and i == steps - 1:
+                before_last()
             fn()
             if os.environ.get("RSB_STEP_MARKS"):
                 m = torch.cuda.Event(enable_timing=True)
@@ -443,12 +460,29 @@ def run_ours(workload, args, rank, local_rank, world, dev, full):
         reserved = now
         step_resident()
         step_resident()
+
+    def restore_initial_state():
+        # in place and in stream order: a captured graph keeps reading / writing these same tensors
+        for k, v in model.state_dict().items():
+            v.copy_(initial_state[k])
+        for st in opt.state.values():
+            if st.get("momentum_buffer") is not None:
+                st["momentum_buffer"].zero_()       # SGD's first step with a zero buffer is its step without one
+        torch.manual_seed(rank)
+        np.random.seed(rank)
+
     clocks = ClockSampler(local_rank)
     if full and rank == 0 and not os.environ.get("RSB_NO_CLOCKS"):
         clocks.start()
     _native.reset_launch_count()
     mallocs0 = torch.cuda.memory_stats(dev).get("num_device_alloc", 0)
-    ms_step = timed(step_resident, args.steps)
+    ms_step = timed(step_resident, args.steps, before_last=restore_initial_state if initial_state is not None else None)
+    outputs = None
+    if args.dump_outputs:
+        flat = lambda ts: torch.cat([t.detach().reshape(-1) for t in ts]).float().cpu().numpy()
+        outputs = {"loss": last["loss"].detach().float().cpu().numpy(),
+                   "grads": flat([p.grad if p.grad is not None else torch.zeros_like(p) for p in params]),
+                   "params": flat(params)}
     device_allocs = torch.cuda.memory_stats(dev).get("num_device_alloc", 0) - mallocs0      # cudaMalloc calls inside (diagnostic)
     launches = _native.launch_count() if gstep is None else gstep.launches_per_step * args.steps   # replays bypass the counter
     clk = clocks.stop() if (full and rank == 0) else None
@@ -480,12 +514,12 @@ def run_ours(workload, args, rank, local_rank, world, dev, full):
         knn_work = [int(v) for v in ctr.tolist()]
 
     clouds_total = wl["clouds"] * world
-    res = {"workload": wl["name"], "value": clouds_total / (ms_step * 1e-3), "ms_per_step": ms_step,
+    res = {"key": workload, "workload": wl["name"], "value": clouds_total / (ms_step * 1e-3), "ms_per_step": ms_step,
            "e2e": {"value": clouds_total / (ms_e2e * 1e-3), "unit": "clouds/s", "ms_per_step": ms_e2e,
                    "h2d_bytes_per_step": h2d_bytes, "d2h_bytes_per_step": 4},
            "gpu_launches": int(launches), "clocks": clk, "per_entry": per_entry, "knn_work": knn_work, "ms_serial": ms_serial,
            "host_issue_ms": {k: (v if isinstance(v, list) else round(v, 3)) for k, v in host_issue.items()},
-           "device_allocs": int(device_allocs), "cuda_graph": gstep is not None, "graph_error": graph_error}
+           "device_allocs": int(device_allocs), "cuda_graph": gstep is not None, "graph_error": graph_error, "outputs": outputs}
     del model, opt, fg, devin, gstep
     torch.cuda.empty_cache()
     return res
@@ -617,6 +651,7 @@ def main():
     ap.add_argument("--threads", type=int, default=1)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-secondary", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None)
     args = ap.parse_args()
 
     rank = int(os.environ.get("RANK", 0))
@@ -665,6 +700,14 @@ def main():
         if world > 1:
             dist.destroy_process_group()
         return
+    if args.dump_outputs:
+        arrays = {f"{res['key']}_{name}": a for res in (r, second) if res is not None for name, a in res["outputs"].items()}
+        total = sum(a.nbytes for a in arrays.values())
+        if total > DUMP_LIMIT_BYTES:
+            raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT_BYTES} byte limit")
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in arrays.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
 
     rooflines, entry_share = build_rooflines(r["per_entry"], r["knn_work"], r["ms_serial"] or r["ms_per_step"], args.steps, args.workload)
     dom = max(r["per_entry"].items(), key=lambda kv: kv[1]["ms"]) if r["per_entry"] else None

@@ -1,12 +1,15 @@
-"""Segmentation input pipeline (SURVEY.md 8 f1): the numpy restatement against the UNMODIFIED reference functions where they
-are deterministic (CPU, build container only), and the device pipeline against the restatement (GPU)."""
-import os
+"""Segmentation input pipeline (SURVEY.md 8 f1): the numpy restatement against the recorded outputs of the UNMODIFIED reference
+functions where they are deterministic (CPU), and the device pipeline against the restatement (GPU)."""
+import contextlib
 
 import numpy as np
 import pytest
 import torch
 
 from oracle import datapath_ref as D
+from tests.reference_golden import Reference
+
+REF = Reference("reference_datapath")
 
 
 def _scan(n, seed):
@@ -23,33 +26,43 @@ def _scan(n, seed):
     return p, feat, label
 
 
+@contextlib.contextmanager
+def _reference(module):
+    """the UNMODIFIED reference module while its outputs are being recorded, None otherwise"""
+    if not REF.recording:
+        yield None
+        return
+    from oracle import ref_loader as RL
+    with RL.RefTree("seg") as t:
+        yield t.imp(module)
+
+
 def test_restatement_matches_reference_functions():
     """fnv_hash_vec bit for bit; voxelize as SETS of voxels / members (the reference's argsort is unstable, so the member it
-    picks inside a voxel is implementation-defined); needs /root/reference."""
-    from oracle import ref_loader as RL
-    if not RL.available():
-        pytest.skip("/root/reference not present (GPU box)")
+    picks inside a voxel is implementation-defined)."""
     coord, _, _ = _scan(50000, 0)
-    with RL.RefTree("seg") as t:
-        V = t.imp("modules.voxelize_utils")
-        disc = np.floor((coord - coord.min(0)) / np.float32(0.04))
-        assert np.array_equal(V.fnv_hash_vec(disc), D.fnv_hash_vec(disc))
-        ref_sort, ref_count = V.voxelize(coord - coord.min(0), 0.04, mode=1)
-        my_sort, my_count = D.voxelize(coord - coord.min(0), 0.04, mode=1)
+    c0 = coord - coord.min(0)
+    disc = np.floor(c0 / np.float32(0.04))
+    with _reference("modules.voxelize_utils") as V:
+        REF.equal("fnv_hash_vec", D.fnv_hash_vec(disc), lambda: V.fnv_hash_vec(disc))
+        ref_count = REF.array("voxelize.count", lambda: V.voxelize(c0, 0.04, mode=1)[1].astype(np.uint16))
+        my_sort, my_count = D.voxelize(c0, 0.04, mode=1)
         assert np.array_equal(ref_count, my_count)
         s = np.cumsum(np.insert(ref_count, 0, 0))
-        for v in np.random.RandomState(1).randint(0, len(ref_count), 200):        # same members per voxel, any order
-            assert set(ref_sort[s[v]:s[v + 1]]) == set(my_sort[s[v]:s[v + 1]])
+        voxels = np.random.RandomState(1).randint(0, len(ref_count), 200)
+        # same members per voxel, any order
+        members = lambda order: np.concatenate([np.sort(order[s[v]:s[v + 1]]) for v in voxels])
+        assert np.array_equal(REF.array("voxelize.members", lambda: members(V.voxelize(c0, 0.04, mode=1)[0])), members(my_sort))
         np.random.seed(3)
-        pick = V.voxelize(coord - coord.min(0), 0.04)
+        pick = REF.array("voxelize.pick", lambda: V.voxelize(c0, 0.04).astype(np.uint16))
         keys = D.fnv_hash_vec(disc)
         assert len(pick) == len(ref_count) and len(np.unique(keys[pick])) == len(pick)
         # hash_type='ravel': keys bit for bit (also for a cloud that does not start at the origin), same voxel sizes
-        for c in (coord - coord.min(0), coord - np.float32(1.7)):
+        for i, c in enumerate((c0, coord - np.float32(1.7))):
             d = np.floor(c / np.float32(0.04))
-            assert np.array_equal(V.ravel_hash_vec(d), D.ravel_hash_vec(d))
-        rs, rc = V.voxelize(coord - coord.min(0), 0.04, hash_type='ravel', mode=1)
-        ms, mc = D.voxelize(coord - coord.min(0), 0.04, hash_type='ravel', mode=1)
+            REF.equal(f"ravel_hash_vec[{i}]", D.ravel_hash_vec(d), lambda: V.ravel_hash_vec(d))
+        rc = REF.array("voxelize_ravel.count", lambda: V.voxelize(c0, 0.04, hash_type='ravel', mode=1)[1].astype(np.uint16))
+        ms, mc = D.voxelize(c0, 0.04, hash_type='ravel', mode=1)
         assert np.array_equal(rc, mc) and np.array_equal(np.sort(rc), np.sort(ref_count))
 
 
@@ -57,36 +70,47 @@ def test_scene_crop_plan_matches_reference_data_process():
     """data_load's voxel parts and data_process's covering crops (segmentation/tool/test_s3dis.py:114-159) against the
     UNMODIFIED reference functions, same numpy seed.  Rows whose fp32 squared distances to a seed tie exactly come out of the
     reference's unstable argsort in either order (seen: a swapped pair in 13 of 117 crops), so crops are compared as row sets plus
-    position-wise agreement; needs /root/reference."""
+    position-wise agreement.  The reference's crop coordinates and features are kept for a sample of crops."""
     import types
-    from oracle import ref_loader as RL
-    if not RL.available():
-        pytest.skip("/root/reference not present (GPU box)")
     coord, feat, _ = _scan(30000, 4)
-    with RL.RefTree("seg") as t:
-        T = t.imp("tool.test_s3dis")
-        T.args = types.SimpleNamespace(voxel_size=0.04, voxel_max=3000, data_norm='mean', color_mean=None, color_std=None)
-        idx_sort, count = T.voxelize(coord - np.min(coord, 0), 0.04, mode=1)
-        ref_parts = [idx_sort[np.cumsum(np.insert(count, 0, 0)[0:-1]) + i % count] for i in range(count.max())]
-        my_parts = D.scene_parts(coord, 0.04)
-        assert len(ref_parts) == len(my_parts) and len(my_parts) >= 2
+    my_parts = D.scene_parts(coord, 0.04)
+    with _reference("tool.test_s3dis") as T:
+        def ref_parts():
+            T.args = types.SimpleNamespace(voxel_size=0.04, voxel_max=3000, data_norm='mean', color_mean=None, color_std=None)
+            idx_sort, count = T.voxelize(coord - np.min(coord, 0), 0.04, mode=1)
+            return [idx_sort[np.cumsum(np.insert(count, 0, 0)[0:-1]) + i % count] for i in range(count.max())]
+        # same voxels in the same order; which MEMBER is i-th in a voxel is the unstable argsort's choice
+        assert np.array_equal(REF.array("scene_parts.sizes", lambda: [len(p) for p in ref_parts()]), [len(p) for p in my_parts])
+        assert len(my_parts) >= 2
         assert sorted(np.unique(np.concatenate(my_parts))) == list(range(coord.shape[0]))      # every point is in some part
-        for a, b in zip(ref_parts, my_parts):
-            # same voxels in the same order; which MEMBER is i-th in a voxel is the unstable argsort's choice
-            assert a.shape == b.shape
-        np.random.seed(9)
-        ri, rc, rf, ro = T.data_process(coord.copy(), feat.copy(), my_parts)
-        np.random.seed(9)
-        mi, mc, mf, mo = D.data_process(coord, feat, my_parts, 3000)
-    assert ro == mo and len(ri) == len(mi) and len(mi) > len(my_parts)
+
+        ref = []
+
+        def ref_process():
+            if not ref:
+                np.random.seed(9)
+                ref.append(T.data_process(coord.copy(), feat.copy(), my_parts))
+            return ref[0]
+        ro = [int(o) for o in REF.array("data_process.offsets", lambda: ref_process()[3])]
+        sample = np.sort(np.random.RandomState(2).choice(len(ro), 4, replace=False))
+        cut = np.cumsum([ro[j] for j in sample])[:-1]
+        kept = lambda k, dtype: dict(zip(sample, np.split(REF.array(f"data_process.{k}_sample", lambda: np.concatenate(
+            [ref_process()[("rows", "coord", "feat").index(k)][j] for j in sample]).astype(dtype)), cut)))
+        ri, rc, rf = kept("rows", np.uint16), kept("coord", np.float32), kept("feat", np.float32)
+    np.random.seed(9)
+    mi, mc, mf, mo = D.data_process(coord, feat, my_parts, 3000)
+    assert ro == mo and len(mi) > len(my_parts)
     same = 0
-    for a, b, ca, cb, fa, fb in zip(ri, mi, rc, mc, rf, mf):
-        assert np.array_equal(np.sort(a), np.sort(b))                  # the same rows in every crop, crop after crop
-        eq = a == b
-        assert eq.mean() > 0.99                                        # in the same order except inside distance ties
-        assert np.array_equal(ca[eq], cb[eq]) and np.array_equal(fa[eq], fb[eq])
-        same += int(eq.all())
-    assert same >= len(ri) // 2                                      # most crops have no tie at all
+    for j, b in enumerate(mi):
+        # the same rows in every crop, crop after crop
+        REF.equal(f"data_process.rows_set[{j}]", np.sort(b), lambda: np.sort(ref_process()[0][j]))
+        same += REF.same(f"data_process.rows[{j}]", b, lambda: ref_process()[0][j])
+        if j in ri:
+            a = ri[j]
+            eq = a == b
+            assert eq.mean() > 0.99                                    # in the same order except inside distance ties
+            assert np.array_equal(rc[j][eq], mc[j][eq]) and np.array_equal(rf[j][eq], mf[j][eq])
+    assert same >= len(mi) // 2                                      # most crops have no tie at all
 
 
 @pytest.mark.gpu

@@ -1,5 +1,5 @@
 """GPU parity suite (-m gpu): every CUDA operator, called through the C-ABI, against the CPU oracle on the same
-seeded inputs (bit-exact for indices), against the reference's own CUDA kernels (oracle/_ref) when present,
+seeded inputs (bit-exact for indices), against the recorded outputs of the reference's own CUDA kernels,
 and size-independent properties at the full BASELINE sizes."""
 import math
 import os
@@ -439,6 +439,7 @@ def test_dense_knn_large_clouds_grid_route_matches_allpairs_and_reference(k):
     from repsurf_b200 import _native as N
     from repsurf_b200.cls import pointops as P
     from tests import refcuda as R
+    from tests.reference_golden import Reference
     g = torch.Generator().manual_seed(77 + k)
     b, n, m = 3, 6000, 1500
     xyz = torch.rand(b, n, 3, generator=g).to(cuda)
@@ -453,6 +454,6 @@ def test_dense_knn_large_clouds_grid_route_matches_allpairs_and_reference(k):
     d2 = torch.empty(b, m, k, device=cuda)
     N.call("rsb_knnquery_heap_dense", b, n, m, k, xyz, new_xyz, aph, d2)
     assert torch.equal(goth, aph)
-    if R.available("cls"):
-        assert torch.equal(got, R.knn_dense(k, xyz, new_xyz))
-        assert torch.equal(goth, R.knn_heap_dense(k, xyz, new_xyz)[0])
+    REF = Reference("reference_cuda")
+    REF.equal(f"knn_dense_large[{k}]", got, lambda: R.knn_dense(k, xyz, new_xyz))
+    REF.equal(f"knn_heap_dense_large[{k}]", goth, lambda: R.knn_heap_dense(k, xyz, new_xyz)[0])

@@ -1,5 +1,5 @@
 """subtraction / aggregation (the PointTransformer operators of the shared pointops package, SURVEY.md 8 f4): the C oracle on
-the CPU against plain tensor formulas; the sm_100a kernels against the oracle and against the reference's own CUDA kernels."""
+the CPU against plain tensor formulas; the sm_100a kernels against the oracle and against the recorded outputs of the reference's own CUDA kernels."""
 import numpy as np
 import pytest
 import torch
@@ -50,9 +50,13 @@ def test_oracle_matches_tensor_formulas(n, ns, c, w_c, seed):
 def test_kernels_match_oracle_and_reference_cuda(n, ns, c, w_c, seed):
     from repsurf_b200.seg import pointops as P
     from tests import refcuda as R
+    from tests.reference_golden import Reference, sample_rows
+    REF = Reference("reference_cuda")
+    case = f"[{n},{ns},{c},{w_c},{seed}]"
     cuda = torch.device("cuda")
     inp, in2, pos, w, idx, go3, go2 = [t.to(cuda) for t in _case(n, ns, c, w_c, seed)]
     small = n <= 2000
+    rows = torch.from_numpy(sample_rows(n, 128)).to(cuda)        # reference gradients are kept for a sample of rows
     # ---- subtraction
     a = inp.clone().requires_grad_(True)
     b = in2.clone().requires_grad_(True)
@@ -60,10 +64,11 @@ def test_kernels_match_oracle_and_reference_cuda(n, ns, c, w_c, seed):
     if small:
         assert torch.equal(out.cpu(), O.subtraction_fwd(inp.cpu(), in2.cpu(), idx.cpu()))            # bit-exact
     out.backward(go3)
-    if R.available("seg"):
-        assert torch.equal(out.detach(), R.subtraction_fwd(inp, in2, idx))                           # bit-exact vs reference CUDA
-        r1, r2 = R.subtraction_bwd(go3, idx)
-        assert torch.allclose(a.grad, r1, rtol=1e-5, atol=1e-5) and torch.allclose(b.grad, r2, rtol=1e-5, atol=1e-5)
+    REF.equal("subtraction_fwd" + case, out, lambda: R.subtraction_fwd(inp, in2, idx))               # bit-exact vs reference CUDA
+    r1 = REF.array("subtraction_bwd.grad1_rows" + case, lambda: R.subtraction_bwd(go3, idx)[0][rows])
+    r2 = REF.array("subtraction_bwd.grad2_rows" + case, lambda: R.subtraction_bwd(go3, idx)[1][rows])
+    assert torch.allclose(a.grad[rows].cpu(), torch.from_numpy(r1), rtol=1e-5, atol=1e-5)
+    assert torch.allclose(b.grad[rows].cpu(), torch.from_numpy(r2), rtol=1e-5, atol=1e-5)
     if small:
         g1, g2 = O.subtraction_bwd(go3.cpu(), idx.cpu())
         assert torch.allclose(a.grad.cpu(), g1, rtol=1e-5, atol=1e-5) and torch.allclose(b.grad.cpu(), g2, rtol=1e-5, atol=1e-5)
@@ -75,11 +80,12 @@ def test_kernels_match_oracle_and_reference_cuda(n, ns, c, w_c, seed):
     if small:
         assert torch.equal(out.cpu(), O.aggregation_fwd(inp.cpu(), pos.cpu(), w.cpu(), idx.cpu()))  # bit-exact (same fma chain)
     out.backward(go2)
-    if R.available("seg"):
-        assert torch.equal(out.detach(), R.aggregation_fwd(inp, pos, w, idx))                        # bit-exact vs reference CUDA
-        r_in, r_pos, r_w = R.aggregation_bwd(inp, pos, w, idx, go2)
-        assert torch.equal(p.grad, r_pos)
-        assert torch.allclose(x.grad, r_in, rtol=1e-5, atol=1e-5) and torch.allclose(ww.grad, r_w, rtol=1e-4, atol=1e-4)
+    REF.equal("aggregation_fwd" + case, out, lambda: R.aggregation_fwd(inp, pos, w, idx))            # bit-exact vs reference CUDA
+    REF.equal("aggregation_bwd.grad_pos" + case, p.grad, lambda: R.aggregation_bwd(inp, pos, w, idx, go2)[1])
+    r_in = REF.array("aggregation_bwd.grad_in_rows" + case, lambda: R.aggregation_bwd(inp, pos, w, idx, go2)[0][rows])
+    r_w = REF.array("aggregation_bwd.grad_w_rows" + case, lambda: R.aggregation_bwd(inp, pos, w, idx, go2)[2][rows])
+    assert torch.allclose(x.grad[rows].cpu(), torch.from_numpy(r_in), rtol=1e-5, atol=1e-5)
+    assert torch.allclose(ww.grad[rows].cpu(), torch.from_numpy(r_w), rtol=1e-4, atol=1e-4)
     if small:
         g_in, g_pos, g_w = O.aggregation_bwd(inp.cpu(), pos.cpu(), w.cpu(), idx.cpu(), go2.cpu())
         assert torch.equal(p.grad.cpu(), g_pos)

@@ -44,15 +44,16 @@ def test_grid_knn_k32_on_a_million_point_segment_matches_all_pairs():
 def test_grid_knn_k32_matches_reference_cuda_on_one_large_segment():
     from repsurf_b200.seg import pointops as P
     from tests import refcuda as R
-    if not R.available("seg"):
-        pytest.skip("oracle/_ref/libref_pointops_seg.so not built")
+    from tests.reference_golden import Reference, sample_rows
+    REF = Reference("reference_cuda")
     n, k = 200_000, 32
     xyz = _room(n, 1).to(cuda)
     off = torch.tensor([n], dtype=torch.int32, device=cuda)
     idx, dist = P.knnquery(k, xyz, xyz, off, off)
-    ridx, rd2 = R.knn_packed(k, xyz, xyz, off, off)
-    assert torch.equal(idx, ridx)
-    assert torch.equal(dist, torch.sqrt(rd2)) or float((dist - torch.sqrt(rd2)).abs().max()) < 1e-6
+    REF.equal("knn_packed_scene.idx", idx, lambda: R.knn_packed(k, xyz, xyz, off, off)[0])
+    rows = torch.from_numpy(sample_rows(n, 512)).to(cuda)
+    rd2 = torch.from_numpy(REF.array("knn_packed_scene.dist2_rows", lambda: R.knn_packed(k, xyz, xyz, off, off)[1][rows])).to(cuda)
+    assert torch.equal(dist[rows], torch.sqrt(rd2)) or float((dist[rows] - torch.sqrt(rd2)).abs().max()) < 1e-6
 
 
 def test_median_filter_matches_torch_median():
